@@ -73,7 +73,7 @@ SH_C = {"c1": 1, "c2": 3, "c3": 4, "c4": 4, "c5": 4}
 def parse():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=50)
+    ap.add_argument("--steps", type=int, default=50, help="steps in each of the five timed loops")
     ap.add_argument("--warmup", type=int, default=5)
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--workload", default="c3", choices=list(SH_C))
@@ -92,6 +92,8 @@ def parse():
                     help="N>1: all-reduce the whole flat gradient buffer instead of the rows some view touched")
     ap.add_argument("--plain-grad-buffer", action="store_true",
                     help="N>1: do not allocate the all-reduce operand with ncclMemAlloc / register it")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed loops, write what their last step computed to DIR/<name>.npy (rank 0)")
     return ap.parse_args()
 
 
@@ -411,6 +413,27 @@ class Workload:
 
     def step(self):
         self.vpr.step(self.n_views, self.render_and_backward)
+
+
+DUMP_GRAD_ROWS = 131072  # Gaussians whose gradient rows --dump-outputs writes (all of them when the scene is smaller)
+
+
+def dump_outputs(out_dir, w):
+    """What the timed step hands its caller, as float32 .npy files: the last rendered view's image and the all-reduced
+    gradient of every parameter.  The gradients are a fixed seeded sample of DUMP_GRAD_ROWS Gaussians (their indices in
+    grad_rows.npy), which keeps the files under 64 MB at the 1M-Gaussian workloads."""
+    import numpy as np
+
+    torch.cuda.synchronize()
+    os.makedirs(out_dir, exist_ok=True)
+    N = w.scene.N
+    rows = torch.randperm(N, generator=torch.Generator().manual_seed(0))[:DUMP_GRAD_ROWS].sort().values
+    arrays = {"rgb": w.last["rgb"].detach(), "grad_rows": rows.double()}
+    for name, g in w.vpr.grad_views.items():
+        if name != "touched":
+            arrays["grad_" + name] = g.detach()[rows.to(g.device)]
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.cpu().numpy())
 
 
 def timed_loops(args, step, barrier, world, dev, n_loops=3, sampler=None, rank=0):
@@ -793,6 +816,8 @@ def run_ours(args):
     runs = timed_loops(args, step, barrier, world, dev, N_LOOPS, sampler, rank)
     all_runs_ms = [r[0] for r in runs]
     ms_max, mark0, mark1 = sorted(runs, key=lambda r: r[0])[N_LOOPS // 2]
+    if args.dump_outputs and rank == 0:  # before anything below runs the step again or all-reduces its gradients
+        dump_outputs(args.dump_outputs, w)
     if w.async_count:  # no view of the timed loops may have been truncated: the blocking check of every context
         from gsgen_b200._lib import TileListOverflow
         from gsgen_b200.rasterizer import view_stats

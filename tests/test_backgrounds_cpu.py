@@ -1,5 +1,6 @@
 """Background models (gsgen_b200/backgrounds.py) against the reference's OWN classes (gs/backgrounds.py compiled out of
-the file with `ast` in the dev container; skipped where /root/reference is absent) draw for draw, and their wiring into
+the file with `ast` where the reference is at $GSB200_REFERENCE; elsewhere against their draws stored in
+tests/golden/backgrounds_ref.npz) draw for draw, and their wiring into
 the trainer-facing renderer (`cfg.background` -> setup_bg, `.bg`, train / eval, checkpoint `bg` state)."""
 import ast
 import os
@@ -10,49 +11,57 @@ import torch
 import torch.nn as nn
 
 from gsgen_b200 import backgrounds as B
-
-REF = "/root/reference/gs/backgrounds.py"
+from tests.util import RefValues
 
 
 class Cfg(dict):
     __getattr__ = dict.__getitem__
 
 
-def _ref_classes():
-    if not os.path.exists(REF):
-        pytest.skip("reference sources not present")
+def _ref_classes(rv):
     from einops import repeat
 
+    path = os.path.join(rv.src, "gs", "backgrounds.py")
     ns = {"torch": torch, "nn": nn, "random": random, "repeat": repeat, "tcnn_capable": False}
-    tree = ast.parse(open(REF).read())
+    tree = ast.parse(open(path).read())
     for node in tree.body:
         if isinstance(node, ast.ClassDef):
-            exec(compile(ast.Module(body=[node], type_ignores=[]), REF, "exec"), ns)
+            exec(compile(ast.Module(body=[node], type_ignores=[]), path, "exec"), ns)
     return ns
 
 
 @pytest.mark.parametrize("kind,extra", [("random", dict(range=[0.2, 0.9])), ("fixed", dict(color=[0.1, 0.5, 0.9])),
                                         ("random", dict(range=[0.0, 1.0], random_aug=True, random_aug_prob=0.5))])
 def test_backgrounds_match_reference_draw_for_draw(kind, extra):
-    ns = _ref_classes()
+    rv = RefValues("backgrounds_ref")
     cfg = Cfg(type=kind, device="cpu", random_aug=False, random_aug_prob=0.0)
     cfg.update(extra)
-    ref = {"random": ns["RandomBackground"], "fixed": ns["FixedBackground"]}[kind](cfg)
+    ref = None
+    if rv.live:
+        ns = _ref_classes(rv)
+        ref = {"random": ns["RandomBackground"], "fixed": ns["FixedBackground"]}[kind](cfg)
     ours = B.make_background(cfg)
-    dirs = torch.randn(5, 7, 3)
-    for mode in (True, False, True):
-        ref.train(mode); ours.train(mode)
-        for _ in range(6):
-            random.seed(11); torch.manual_seed(11)
-            a = ref(dirs)
-            random.seed(11); torch.manual_seed(11)
-            b = ours(dirs)
+    dirs = torch.randn(5, 7, 3, generator=torch.Generator().manual_seed(5))
+    tag = f"{kind}_{'_'.join(f'{k}={v}' for k, v in sorted(extra.items()))}"
+
+    def draw(model):
+        random.seed(11); torch.manual_seed(11)
+        return model(dirs)
+
+    for m, mode in enumerate((True, False, True)):
+        ours.train(mode)
+        if ref is not None:
+            ref.train(mode)
+        for i in range(6):
+            a = torch.from_numpy(rv(f"{tag}_{m}_{i}", lambda: draw(ref)))
+            b = draw(ours)
             assert a.shape == b.shape == (5, 7, 3) and torch.equal(a, b)
     if kind == "fixed":  # the colour is a parameter: gradient of sum(bg * w) is the sum of w over the pixels
         w = torch.randn(5, 7, 3)
         (ours(dirs) * w).sum().backward()
         assert torch.allclose(ours.bg_color.grad, w.sum(dim=(0, 1)))
-        assert set(ours.state_dict()) == set(ref.state_dict()) == {"bg_color"}
+        assert set(ours.state_dict()) == set(rv(f"{tag}_state", lambda: sorted(ref.state_dict()))) == {"bg_color"}
+    rv.save()
 
 
 def test_learned_const_and_unknown_types():

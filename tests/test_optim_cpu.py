@@ -1,17 +1,16 @@
 """CPU checks of the optimizer row (SURVEY §8(f)-3): the Adam arithmetic of `k_adam_flat` (host build of
 gsb200_math.cuh) against torch.optim.Adam as the reference configures it (eps 1e-15, per-field lr), and the restated
-learning-rate schedules against utils/schedulers.py (imported from /root/reference when it is mounted, pinned values
-otherwise)."""
+learning-rate schedules against utils/schedulers.py (imported from $GSB200_REFERENCE when set, otherwise the values it
+computed, tests/golden/schedulers_ref.npz)."""
 import ctypes
 import math
-import os
 import sys
 
 import pytest
 import torch
 
 from gsgen_b200 import optim
-from tests.util import fp
+from tests.util import RefValues, fp
 
 
 def test_adam_arithmetic_matches_torch(hostmath):
@@ -73,22 +72,26 @@ def test_lr_schedules_pinned(key):
     assert optim.make_scheduler(0.003, 15000)(1234) == 0.003
 
 
-@pytest.mark.skipif(not os.path.exists("/root/reference/utils/schedulers.py"), reason="reference not mounted")
 def test_lr_schedules_match_reference_module():
-    sys.path.insert(0, "/root/reference")
-    try:
-        import importlib
-        ref = importlib.import_module("utils.schedulers")
-    finally:
-        sys.path.pop(0)
+    rv = RefValues("schedulers_ref")
+    ref = None
+    if rv.live:
+        sys.path.insert(0, rv.src)
+        try:
+            import importlib
+            ref = importlib.import_module("utils.schedulers")
+        finally:
+            sys.path.pop(0)
     for kind in ("exp", "cosine", "nothing"):
         for (a, b, steps) in ((0.005, 3e-5, 15000), (0.003, 0.001, 15000), (1e-4, 1e-6, 777)):
             ours = optim.lr_schedulers[kind](steps, a, b)
-            theirs = ref.lr_schedulers[kind](steps, a, b)
+            theirs = ref.lr_schedulers[kind](steps, a, b) if ref else None
             for step in (0, 1, 13, steps // 3, steps - 1, steps, steps + 50 if kind != "cosine" else steps):
-                assert math.isclose(ours(step), float(theirs(step)), rel_tol=1e-12), (kind, a, b, steps, step)
+                want = float(rv(f"{kind}_{a}_{b}_{steps}_{step}", lambda: float(theirs(step))))
+                assert math.isclose(ours(step), want, rel_tol=1e-12), (kind, a, b, steps, step)
     # warm-up branch
     ours = optim.exp_decay(1000, 1e-2, 1e-4, warmup_steps=100)
-    theirs = ref.exp_decay(1000, 1e-2, 1e-4, warmup_steps=100)
+    theirs = ref.exp_decay(1000, 1e-2, 1e-4, warmup_steps=100) if ref else None
     for step in (0, 50, 99, 100, 500):
-        assert math.isclose(ours(step), float(theirs(step)), rel_tol=1e-12)
+        assert math.isclose(ours(step), float(rv(f"warmup_{step}", lambda: float(theirs(step)))), rel_tol=1e-12)
+    rv.save()

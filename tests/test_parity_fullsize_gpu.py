@@ -11,38 +11,32 @@ Two tests per configuration:
 
 Tolerances are north_star's: images 1e-4 abs, gradients 1e-3 rel (tests/util.py::assert_grad_close).  Every pixel above
 1e-4 must be explained by `tests/util.py::classify_image_diff` (threshold flip shown by the oracle's margin map, or
-reference-side fp32 rounding shown by the fp64 arbiter); zero unexplained pixels.  The classification counts are written
-to gpurun_out/parity_fullsize.json (copied to profiles/ by hand)."""
+reference-side fp32 rounding shown by the fp64 arbiter); zero unexplained pixels.  Where `oracle/_ref/_gs.so` has not been built, the same comparisons run against a fixed
+sample of the extension's outputs recorded on a B200 (tests/golden/parity_*.npz; tests/util.py::RefGolden).  The
+classification counts are written to $GSB200_PARITY_REPORT when that is set."""
 import json
 import os
-import sys
 
 import pytest
 import torch
 
 from gsgen_b200.scenes import make_scene
-from tests.util import ROOT, assert_grad_close, classify_image_diff, ocam_of
+from tests.util import RefGolden, load_ref_ext, ocam_of
 
 pytestmark = pytest.mark.gpu
 DEV = "cuda"
-REF_DIR = os.path.join(ROOT, "oracle", "_ref")
-REPORT = os.path.join(ROOT, "gpurun_out", "parity_fullsize.json")
+REPORT = os.environ.get("GSB200_PARITY_REPORT")
 
 
 @pytest.fixture(scope="module")
 def ref_gs():
-    if not os.path.exists(os.path.join(REF_DIR, "_gs.so")):
-        pytest.skip("reference extension oracle/_ref/_gs.so not built")
-    sys.path.insert(0, REF_DIR)
-    try:
-        import _gs
-    except Exception as e:  # pragma: no cover
-        pytest.skip(f"reference extension not loadable: {e}")
-    return _gs
+    return load_ref_ext()
 
 
 def _dump(cfg, test, rows):
-    os.makedirs(os.path.dirname(REPORT), exist_ok=True)
+    if not REPORT:
+        return
+    os.makedirs(os.path.dirname(os.path.abspath(REPORT)), exist_ok=True)
     data = {}
     if os.path.exists(REPORT):
         try:
@@ -70,6 +64,8 @@ def test_ops_fullsize_vs_reference_extension(ref_gs, oracle_mod, cfg):
     from gsgen_b200.culling import tile_culling_aabb_count
     from gsgen_b200.renderer import project_gaussians
 
+    R = RefGolden(f"parity_ops_{cfg}", ref_gs)
+    live = R.live
     sc, cam, c2w_cpu = _scene(cfg)
     sc = sc.to(DEV)
     c2w = c2w_cpu.to(DEV)
@@ -82,8 +78,9 @@ def test_ops_fullsize_vs_reference_extension(ref_gs, oracle_mod, cfg):
     mask = torch.zeros(sc.N, dtype=torch.bool, device=DEV)
     rmask = torch.zeros(sc.N, dtype=torch.bool, device=DEV)
     _backend.culling_gaussian_bsphere(sc.mean, sc.qvec, sc.svec, normals, pts, mask, 6.0)
-    ref_gs.culling_gaussian_bsphere(sc.mean, sc.qvec, sc.svec, normals, pts, rmask, 6.0)
-    assert torch.equal(mask, rmask)
+    if live:
+        ref_gs.culling_gaussian_bsphere(sc.mean, sc.qvec, sc.svec, normals, pts, rmask, 6.0)
+    R.equal("mask", mask, rmask)
     m, q, s = sc.mean[mask].contiguous(), sc.qvec[mask].contiguous(), sc.svec[mask].contiguous()
     al, col, sh = sc.alpha[mask].contiguous(), sc.color[mask].contiguous(), sc.sh[mask].contiguous()
     m2, c2, _, dp = project_gaussians(m, q, s, c2w, True)
@@ -92,14 +89,14 @@ def test_ops_fullsize_vs_reference_extension(ref_gs, oracle_mod, cfg):
     mk = lambda: (torch.zeros(D, dtype=torch.int32, device=DEV), -torch.ones(th * tw, dtype=torch.int32, device=DEV),
                   -torch.ones(th * tw, dtype=torch.int32, device=DEV))
     ids, start, end = mk()
-    rids, rstart, rend = mk()
     _backend.tile_culling_aabb_start_end(tl, br, ids, start, end, dp, th, tw)
-    ref_gs.tile_culling_aabb_start_end(tl, br, rids, rstart, rend, dp, th, tw)
+    rids, rstart, rend = mk() if live else (ids, None, None)  # stored: the lists below are ours, pinned here
+    if live:
+        ref_gs.tile_culling_aabb_start_end(tl, br, rids, rstart, rend, dp, th, tw)
     torch.cuda.synchronize()
-    assert torch.equal(start, rstart) and torch.equal(end, rend)
-    neq = ids != rids
-    if bool(neq.any()):  # only inside runs of identical (tile, depth) keys
-        assert torch.equal(dp.view(-1)[ids[neq].long()], dp.view(-1)[rids[neq].long()])
+    R.equal("start", start, rstart)
+    R.equal("end", end, rend)
+    R.sorted_ids("ids", ids, dp, rids if live else None)  # only inside runs of identical (tile, depth) keys
     topleft = torch.tensor([-cam.cx / cam.fx, -cam.cy / cam.fy], device=DEV)
     common = (16, th, tw, 1.0 / cam.fx, 1.0 / cam.fy, H, W)
     g = torch.Generator().manual_seed(77)
@@ -115,20 +112,23 @@ def test_ops_fullsize_vs_reference_extension(ref_gs, oracle_mod, cfg):
     o, T = torch.zeros(H, W, 3, device=DEV), torch.ones(H, W, 1, device=DEV)
     ro, rT = torch.zeros(H, W, 3, device=DEV), torch.ones(H, W, 1, device=DEV)
     _backend.tile_based_vol_rendering_start_end_with_T(m2, c2, col, al, start, end, rids, o, topleft, *common, 1e-4, T)
-    ref_gs.tile_based_vol_rendering_start_end_with_T(m2, c2, col, al, start, end, rids, ro, topleft, *common, 1e-4, rT)
+    if live:
+        ref_gs.tile_based_vol_rendering_start_end_with_T(m2, c2, col, al, start, end, rids, ro, topleft, *common, 1e-4,
+                                                         rT)
     torch.cuda.synchronize()
-    classify_image_diff(o, ro, rgb_margin, what="rgb", report=rows)
-    classify_image_diff(T.view(H, W), rT.view(H, W), rgb_margin, what="T", report=rows)
+    R.image("rgb", o, ro, rgb_margin, report=rows)
+    R.image("T", T.view(H, W), rT.view(H, W), rgb_margin, report=rows)
     gz = lambda: (torch.zeros_like(m2), torch.zeros_like(c2), torch.zeros_like(col), torch.zeros_like(al))
     ga_, gb_ = gz(), gz()
-    final = ro.contiguous()
+    final = (ro if live else o).contiguous()  # the reference's forward output where it ran, else ours (pinned above)
     _backend.tile_based_vol_rendering_backward_start_end(m2, c2, col, al, start, end, rids, final, *ga_, gout, topleft,
                                                          *common, 1e-4)
-    ref_gs.tile_based_vol_rendering_backward_start_end(m2, c2, col, al, start, end, rids, final, *gb_, gout, topleft,
-                                                       *common, 1e-4)
+    if live:
+        ref_gs.tile_based_vol_rendering_backward_start_end(m2, c2, col, al, start, end, rids, final, *gb_, gout, topleft,
+                                                           *common, 1e-4)
     torch.cuda.synchronize()
     for a_, b_, n_ in zip(ga_, gb_, ("g_mean2d", "g_cov2d", "g_color", "g_alpha")):
-        rows.append({"what": "rgb " + n_, "rel_l2": assert_grad_close(a_, b_, what="rgb " + n_)})
+        rows.append({"what": "rgb " + n_, "rel_l2": R.grad("rgb " + n_, a_, b_)})
 
     # ---- SH forward / backward at the configuration's degree; c2w passed as the [3,4] tensor (sh_renderer.py:324)
     def sh_margin():
@@ -142,20 +142,23 @@ def test_ops_fullsize_vs_reference_extension(ref_gs, oracle_mod, cfg):
 
     o, ro = torch.zeros(H * W * 3, device=DEV), torch.zeros(H * W * 3, device=DEV)
     _backend.tile_based_vol_rendering_sh(m2, c2, sh, al, start, end, rids, o, topleft, c2w, *common, C, 1e-4)
-    ref_gs.tile_based_vol_rendering_sh(m2, c2, sh, al, start, end, rids, ro, topleft, c2w, *common, C, 1e-4)
+    if live:
+        ref_gs.tile_based_vol_rendering_sh(m2, c2, sh, al, start, end, rids, ro, topleft, c2w, *common, C, 1e-4)
     torch.cuda.synchronize()
-    classify_image_diff(o.view(H, W, 3), ro.view(H, W, 3), sh_margin, sh_exact, what=f"sh rgb C={C}", report=rows)
+    R.image(f"sh rgb C={C}", o.view(H, W, 3), ro.view(H, W, 3), sh_margin, sh_exact, report=rows)
     gz = lambda: (torch.zeros_like(m2), torch.zeros_like(c2), torch.zeros_like(sh), torch.zeros_like(al))
     ga_, gb_ = gz(), gz()
     go = gout.view(-1).contiguous()
-    _backend.tile_based_vol_rendering_backward_sh(m2, c2, sh, al, start, end, rids, ro, *ga_, go, topleft, c2w, *common,
-                                                  C, 1e-4)
-    ref_gs.tile_based_vol_rendering_backward_sh(m2, c2, sh, al, start, end, rids, ro, *gb_, go, topleft, c2w, *common,
-                                                C, 1e-4)
+    _backend.tile_based_vol_rendering_backward_sh(m2, c2, sh, al, start, end, rids, ro if live else o, *ga_, go, topleft,
+                                                  c2w, *common, C, 1e-4)
+    if live:
+        ref_gs.tile_based_vol_rendering_backward_sh(m2, c2, sh, al, start, end, rids, ro, *gb_, go, topleft, c2w, *common,
+                                                    C, 1e-4)
     torch.cuda.synchronize()
     for a_, b_, n_ in zip(ga_, gb_, ("g_mean2d", "g_cov2d", "g_sh", "g_alpha")):
-        rows.append({"what": "sh " + n_, "rel_l2": assert_grad_close(a_, b_, what="sh " + n_)})
+        rows.append({"what": "sh " + n_, "rel_l2": R.grad("sh " + n_, a_, b_)})
     rows.append({"what": "sizes", "N": sc.N, "N_visible": int(mask.sum()), "N_with_dub": D, "H": H, "W": W, "C": C})
+    R.save()
     _dump(cfg, "ops", rows)
 
 
@@ -165,6 +168,10 @@ def test_fused_view_fullsize_vs_reference_pipeline(ref_gs, oracle_mod, cfg):
     from gsgen_b200.culling import tile_culling_aabb_count
     from gsgen_b200.rasterizer import render_view
 
+    from gsgen_b200.backend import _backend
+
+    R = RefGolden(f"parity_fused_{cfg}", ref_gs)
+    live = R.live
     sc, cam, c2w_cpu = _scene(cfg)
     sc = sc.to(DEV)
     c2w = c2w_cpu.to(DEV)
@@ -183,9 +190,11 @@ def test_fused_view_fullsize_vs_reference_pipeline(ref_gs, oracle_mod, cfg):
     mask = aux["mask"]
     # ---- reference pipeline on the same leaves (gs/gaussian_splatting.py:1198-1421 with SHRenderer.forward)
     normals, pts = cam.get_frustum(c2w_cpu)
-    rmask = torch.zeros(sc.N, dtype=torch.bool, device=DEV)
-    ref_gs.culling_gaussian_bsphere(sc.mean, sc.qvec, sc.svec, normals.to(DEV), pts.to(DEV), rmask, 6.0)
-    assert torch.equal(mask, rmask)
+    rmask = None
+    if live:
+        rmask = torch.zeros(sc.N, dtype=torch.bool, device=DEV)
+        ref_gs.culling_gaussian_bsphere(sc.mean, sc.qvec, sc.svec, normals.to(DEV), pts.to(DEV), rmask, 6.0)
+    R.equal("mask", mask, rmask)
     mr, qr, sr = leaf(sc.mean), leaf(sc.qvec), leaf(sc.svec)
     m2, c2, _, dp = oracle_mod.project_gaussians(mr[mask], qr[mask], sr[mask], c2w, True)  # the reference's torch ops
     m2d, c2d, dpd = m2.detach().contiguous(), c2.detach().contiguous(), dp.detach().contiguous()
@@ -200,17 +209,20 @@ def test_fused_view_fullsize_vs_reference_pipeline(ref_gs, oracle_mod, cfg):
     rids = torch.zeros(D, dtype=torch.int32, device=DEV)
     rstart = -torch.ones(th * tw, dtype=torch.int32, device=DEV)
     rend = -torch.ones(th * tw, dtype=torch.int32, device=DEV)
-    ref_gs.tile_culling_aabb_start_end(tl, br, rids, rstart, rend, dpd, th, tw)
+    # (stored: the margin maps below are built on our binning of the same inputs, bit-exact with the reference's: ops test)
+    (ref_gs if live else _backend).tile_culling_aabb_start_end(tl, br, rids, rstart, rend, dpd, th, tw)
     topleft = torch.tensor([-cam.cx / cam.fx, -cam.cy / cam.fy], device=DEV)
     common = (16, th, tw, 1.0 / cam.fx, 1.0 / cam.fy, H, W)
     al, sh = sc.alpha[mask].contiguous(), sc.sh[mask].contiguous()
     ro = torch.zeros(H * W * 3, device=DEV)
-    ref_gs.tile_based_vol_rendering_sh(m2d, c2d, sh, al, rstart, rend, rids, ro, topleft, c2w, *common, C, 1e-4)
-    g_m2, g_c2 = torch.zeros_like(m2d), torch.zeros_like(c2d)
-    g_sh, g_al = torch.zeros_like(sh), torch.zeros_like(al)
-    ref_gs.tile_based_vol_rendering_backward_sh(m2d, c2d, sh, al, rstart, rend, rids, ro, g_m2, g_c2, g_sh, g_al,
-                                                gout.view(-1).contiguous(), topleft, c2w, *common, C, 1e-4)
-    torch.autograd.backward([m2, c2], [g_m2, g_c2])
+    g_m2 = g_sh = g_al = None
+    if live:
+        ref_gs.tile_based_vol_rendering_sh(m2d, c2d, sh, al, rstart, rend, rids, ro, topleft, c2w, *common, C, 1e-4)
+        g_m2, g_c2 = torch.zeros_like(m2d), torch.zeros_like(c2d)
+        g_sh, g_al = torch.zeros_like(sh), torch.zeros_like(al)
+        ref_gs.tile_based_vol_rendering_backward_sh(m2d, c2d, sh, al, rstart, rend, rids, ro, g_m2, g_c2, g_sh, g_al,
+                                                    gout.view(-1).contiguous(), topleft, c2w, *common, C, 1e-4)
+        torch.autograd.backward([m2, c2], [g_m2, g_c2])
     torch.cuda.synchronize()
     # ---- per-Gaussian by-products of the fused front end against the reference's torch stage
     assert torch.allclose(aux["mean2d"].detach()[mask], m2d, rtol=2e-5, atol=1e-6)
@@ -245,12 +257,13 @@ def test_fused_view_fullsize_vs_reference_pipeline(ref_gs, oracle_mod, cfg):
                                                      cfg_o)
         return e, mx
 
-    classify_image_diff(out["rgb"], ro.view(H, W, 3), sh_margin, sh_exact, what=f"fused sh rgb C={C}", report=rows,
-                        exact_self_fn=sh_exact_own)
+    R.image(f"fused sh rgb C={C}", out["rgb"], ro.view(H, W, 3), sh_margin, sh_exact, report=rows,
+            exact_self_fn=sh_exact_own)
     # ---- parameter gradients (north_star: xyz / scale / rot / opacity / SH within 1e-3 rel)
-    full = lambda t, like: torch.zeros_like(like).index_put_((mask,), t)
+    full = lambda t, like: None if t is None else torch.zeros_like(like).index_put_((mask,), t)
     for a_, b_, n_ in ((mg.grad, mr.grad, "g_mean"), (qg.grad, qr.grad, "g_qvec"), (sg.grad, sr.grad, "g_svec"),
                        (ag.grad, full(g_al, sc.alpha), "g_alpha"), (shg.grad, full(g_sh, sc.sh), "g_sh"),
                        (aux["mean2d_grad"][mask], g_m2, "g_mean2d")):
-        rows.append({"what": "fused " + n_, "rel_l2": assert_grad_close(a_, b_, what="fused " + n_)})
+        rows.append({"what": "fused " + n_, "rel_l2": R.grad("fused " + n_, a_, b_)})
+    R.save()
     _dump(cfg, "fused_view", rows)

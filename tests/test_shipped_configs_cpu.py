@@ -2,11 +2,13 @@
 experiment files) drives `gsgen_b200.splatting.GaussianSplattingRenderer` through the trainer's call sequence on the CPU
 (oracle as `render_fn`, brute-force search as `knn_fn`): construction incl. `setup_bg`, `setup_lr` / `set_optimizer`,
 one batch forward + backward + `post_backward`, `auxiliary_loss`, and `densify(step)` / `prune(step)` at
-a step where the config's own gates fire.  The yaml files are read where they lie (/root/reference; skipped elsewhere);
-OmegaConf interpolations (`${device}`, `${max_steps}`) are resolved by hand.  What it pins: no shipped key is
+a step where the config's own gates fire.  The yaml files are read where they lie when $GSB200_REFERENCE names the
+reference (and then written to $GSB200_GOLDEN_OUT/shipped_renderer_configs.json when that is set); elsewhere their parsed
+contents come from tests/golden/shipped_renderer_configs.json.  OmegaConf interpolations (`${device}`, `${max_steps}`) are resolved by hand.  What it pins: no shipped key is
 unsupported or mis-read (densify types official / all / scale / compatness / shrink_then_compatness, the three prune
 rules, penalty schedules, background types) -- the numerical parity of each piece is pinned elsewhere."""
 import glob
+import json
 import os
 
 import pytest
@@ -15,8 +17,11 @@ import yaml
 
 from gsgen_b200.scenes import make_scene
 from tests.test_splatting_cpu import _oracle_render_fn
+from tests.util import GOLDEN
 
-CONF = "/root/reference/conf"
+REF = os.environ.get("GSB200_REFERENCE")
+CONF = os.path.join(REF, "conf") if REF else None
+STORED = os.path.join(GOLDEN, "shipped_renderer_configs.json")
 MAX_STEPS = 5000
 
 
@@ -31,29 +36,36 @@ def _resolve(x):
     return x
 
 
-def _configs():
-    out = []
-    if not os.path.isdir(CONF):
-        return out
+def _read_configs():
+    """{"<file relative to conf/>|<key or empty>": the renderer block as parsed}"""
+    out = {}
     for path in sorted(glob.glob(os.path.join(CONF, "renderer", "*.yaml"))):
-        if isinstance(yaml.safe_load(open(path)), dict):  # (short.yaml is an empty file)
-            out.append((os.path.relpath(path, CONF), None))
+        d = yaml.safe_load(open(path))
+        if isinstance(d, dict):  # (short.yaml is an empty file)
+            out[os.path.relpath(path, CONF) + "|"] = d
     for path in sorted(glob.glob(os.path.join(CONF, "*.yaml"))):
         try:
             d = yaml.safe_load(open(path))
         except Exception:
             continue
         if isinstance(d, dict) and isinstance(d.get("renderer"), dict) and "densify" in d["renderer"]:
-            out.append((os.path.relpath(path, CONF), "renderer"))
+            out[os.path.relpath(path, CONF) + "|renderer"] = d["renderer"]
+    out_dir = os.environ.get("GSB200_GOLDEN_OUT")
+    if out_dir:
+        os.makedirs(out_dir, exist_ok=True)
+        json.dump(out, open(os.path.join(out_dir, os.path.basename(STORED)), "w"), indent=1, sort_keys=True)
     return out
 
 
-@pytest.mark.parametrize("rel,sub", _configs() or [pytest.param(None, None, marks=pytest.mark.skip("no reference conf"))])
+CONFIGS = _read_configs() if CONF and os.path.isdir(CONF) else json.load(open(STORED))
+
+
+# (None, None): no configuration file at all -- the renderer's own defaults (no densify, no prune, no background)
+@pytest.mark.parametrize("rel,sub", [(None, None)] + [(k.split("|")[0], k.split("|")[1] or None) for k in CONFIGS])
 def test_shipped_renderer_config_drives_the_renderer(oracle_mod, rel, sub):
     from gsgen_b200.splatting import GaussianSplattingRenderer
 
-    d = yaml.safe_load(open(os.path.join(CONF, rel)))
-    cfg = _resolve(d[sub] if sub else d)
+    cfg = _resolve(CONFIGS[f"{rel}|{sub or ''}"]) if rel is not None else {}
     if cfg.get("background", {}).get("type") == "mlp":
         cfg["background"] = dict(cfg["background"], type="fixed", color=[0.0, 0.0, 0.0])  # tinycudann: outside the path
     sc = make_scene("c1", N=300, reso=48)

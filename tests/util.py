@@ -1,7 +1,9 @@
 """Shared helpers of the parity tests."""
 import ctypes
+import hashlib
 import os
 import re
+import zlib
 
 import numpy as np
 import torch
@@ -160,3 +162,141 @@ def classify_image_diff(ours, ref, margin_fn, exact_fn=None, atol=IMG_ATOL, what
     assert res.get("flip_max_err", 0.0) <= 8e-3, f"{what}: threshold-flip error larger than one blend step: {res}"
     assert res["flip_explained"] <= max(4, max_flip_frac * epix.numel()), f"{what}: too many flip pixels: {res}"
     return res
+
+
+def load_ref_ext():
+    """The unmodified reference `_gs` extension (oracle/_ref/_gs.so, built by oracle/build_ref.sh from the reference's
+    sources), or None where it has not been built."""
+    import sys
+
+    ref_dir = os.path.join(ROOT, "oracle", "_ref")
+    if not os.path.exists(os.path.join(ref_dir, "_gs.so")):
+        return None
+    if ref_dir not in sys.path:
+        sys.path.insert(0, ref_dir)
+    import _gs
+
+    return _gs
+
+
+class RefGolden:
+    """The reference extension's side of a full-size comparison.
+
+    live (`ext` is the extension): each of its outputs is compared whole, as the reference's own numbers, and a fixed
+    seeded sample of it is kept; save() writes the samples to $GSB200_GOLDEN_OUT/<name>.npz when that is set.  Stored
+    (`ext` is None): the same comparison runs on that sample, read from tests/golden/<name>.npz, against the same
+    elements of ours.  Integer results (masks, tile ranges, sorted ids) are pinned whole by their SHA-256."""
+
+    N_PIX = 384  # sampled pixels per image
+    N_EL = 384  # sampled elements per gradient tensor
+
+    def __init__(self, name, ext):
+        self.name, self.ext, self.rec = name, ext, {}
+        self.z = None if ext is not None else np.load(os.path.join(GOLDEN, name + ".npz"))
+
+    @property
+    def live(self):
+        return self.ext is not None
+
+    def _idx(self, key, n, k):
+        g = torch.Generator().manual_seed(zlib.crc32(f"{self.name}/{key}".encode()))
+        return torch.randperm(n, generator=g)[:min(k, n)].sort().values
+
+    def stored(self, key):
+        return torch.from_numpy(self.z[key])
+
+    @staticmethod
+    def _sha(t):
+        return np.frombuffer(hashlib.sha256(t.detach().cpu().contiguous().numpy().tobytes()).digest(), np.uint8)
+
+    def scalar(self, key, fn):
+        """a number the comparison derives from the reference's output (e.g. an image's scale)"""
+        if self.live:
+            self.rec[key] = np.float64(fn())
+        return float(self.rec[key] if self.live else self.z[key])
+
+    def equal(self, key, ours, ref=None):
+        if self.live:
+            assert torch.equal(ours, ref), key
+            self.rec[key + "_sha"] = self._sha(ref)
+        else:
+            assert np.array_equal(self._sha(ours), self.z[key + "_sha"]), f"{key}: differs from the reference"
+
+    def sorted_ids(self, key, ids, depth, ref=None):
+        """tile-sorted Gaussian ids: equal to the reference's, except inside runs of identical (tile, depth) keys"""
+        idx = self._idx(key, ids.numel(), self.N_EL)
+        if self.live:
+            self.rec[key + "_sha"] = self._sha(ref)
+            self.rec[key] = ref.cpu()[idx].numpy()
+            rids = ref
+        elif np.array_equal(self._sha(ids), self.z[key + "_sha"]):
+            return
+        else:
+            ids, rids = ids[idx.to(ids.device)], self.stored(key).to(ids.device)
+        neq = ids != rids
+        if bool(neq.any()):
+            assert torch.equal(depth.view(-1)[ids[neq].long()], depth.view(-1)[rids[neq].long()]), key
+
+    def image(self, key, ours, ref, margin_fn, exact_fn=None, exact_self_fn=None, **kw):
+        """classify_image_diff (tests/util.py) on the whole image, or on the stored pixels"""
+        H, W = ours.shape[0], ours.shape[1]
+        idx = self._idx(key, H * W, self.N_PIX)
+        if self.live:
+            self.rec[key] = ref.detach().float().cpu().reshape(H * W, -1)[idx].numpy()
+            return classify_image_diff(ours, ref, margin_fn, exact_fn, what=key, exact_self_fn=exact_self_fn, **kw)
+        pick = lambda t: t.detach().cpu().reshape(H * W, -1)[idx].unsqueeze(1)  # [S, 1, channels]: one pixel per row
+        pick_m = lambda m: m.reshape(H * W)[idx].unsqueeze(1)
+
+        def wrap(fn):
+            return None if fn is None else (lambda: (lambda e, m: (pick(e), pick_m(m)))(*fn()))
+
+        return classify_image_diff(pick(ours), self.stored(key).unsqueeze(1), lambda: pick_m(margin_fn()), wrap(exact_fn),
+                                   what=key + " (stored pixels)", exact_self_fn=wrap(exact_self_fn), **kw)
+
+    def grad(self, key, ours, ref=None, rtol=GRAD_RTOL):
+        """assert_grad_close on the whole tensor, or on the stored elements"""
+        idx = self._idx(key, ours.numel(), self.N_EL)
+        if self.live:
+            self.rec[key] = ref.detach().float().cpu().reshape(-1)[idx].numpy()
+            return assert_grad_close(ours, ref, rtol, what=key)
+        return assert_grad_close(ours.detach().cpu().reshape(-1)[idx], self.stored(key), rtol, what=key + " (stored elements)")
+
+    def save(self):
+        out = os.environ.get("GSB200_GOLDEN_OUT")
+        if self.live and out:
+            os.makedirs(out, exist_ok=True)
+            np.savez_compressed(os.path.join(out, self.name + ".npz"), **self.rec)
+
+
+class RefValues:
+    """Values computed by the reference's own Python definitions, for the tests that execute them out of its files.
+
+    Live when $GSB200_REFERENCE names a checkout of the reference: the test executes the definitions (`src` is that
+    directory) and every value passes through; save() writes them to $GSB200_GOLDEN_OUT/<name>.npz when that is set.
+    Otherwise each value comes from tests/golden/<name>.npz, recorded that way."""
+
+    def __init__(self, name):
+        src = os.environ.get("GSB200_REFERENCE")
+        self.name, self.rec = name, {}
+        self.src = src if src and os.path.isdir(src) else None
+        self.z = None if self.live else np.load(os.path.join(GOLDEN, name + ".npz"))
+
+    @property
+    def live(self):
+        return self.src is not None
+
+    def __call__(self, key, fn):
+        """fn() -> the reference's value (live); returned as an ndarray either way"""
+        if self.live:
+            v = fn()
+            self.rec[key] = np.asarray(v.detach().cpu().numpy() if isinstance(v, torch.Tensor) else v)
+            return self.rec[key]
+        return self.z[key]
+
+    def save(self):
+        out = os.environ.get("GSB200_GOLDEN_OUT")
+        if self.live and out:
+            os.makedirs(out, exist_ok=True)
+            path = os.path.join(out, self.name + ".npz")
+            old = dict(np.load(path)) if os.path.exists(path) else {}
+            np.savez_compressed(path, **dict(old, **self.rec))
