@@ -251,7 +251,8 @@ GSB_HD Splat make_splat(const float m2[2], const float cov[4], float alpha) {
   double det = c0 * c3 - c1 * c2;
   double b = 0.5 * (c1 + c2);
   float a = fminf(alpha, kAlphaClamp);
-  bool ok = (det > 0.0) && (c0 > 0.0) && (c3 > 0.0) && (det == det) && (a == a);
+  // NaN alpha must be tested before the clamp: fminf(NaN, 0.99f) is 0.99f
+  bool ok = (det > 0.0) && (c0 > 0.0) && (c3 > 0.0) && (det == det) && (alpha == alpha);
   double A = c3 / det, B = -b / det, Cc = c0 / det;
   double l00 = sqrt(A), l01 = B / l00, l11sq = Cc - l01 * l01;
   ok = ok && (l11sq > 0.0) && (l00 == l00) && (l00 < 1e18) && (l11sq < 1e36);
