@@ -98,6 +98,7 @@ EXPORTS = [
     "gsb200_render_forward", "gsb200_render_backward", "gsb200_view_stats",
     "gsb200_ctx_set_profiling", "gsb200_ctx_get_profile", "gsb200_adam_step", "gsb200_ctx_set_option",
     "gsb200_store_compact", "gsb200_store_append", "gsb200_rows_pack", "gsb200_rows_unpack", "gsb200_knn",
+    "gsb200_estimate_normals", "gsb200_estimate_normals_backward",
 ]
 
 

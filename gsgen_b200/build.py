@@ -15,11 +15,15 @@ HERE = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(HERE, "csrc")
 BUILD = os.path.join(HERE, "_build")
 LIB = os.path.join(HERE, "libgsb200.so")
-SOURCES = ["api.cu", "preprocess.cu", "binning.cu", "composite_fwd.cu", "composite_bwd.cu", "composite_bwd_sh.cu", "optimizer.cu", "store.cu", "knn.cu"]
+SOURCES = ["api.cu", "preprocess.cu", "binning.cu", "composite_fwd.cu", "composite_bwd.cu", "composite_bwd_sh.cu",
+           "optimizer.cu", "store.cu", "knn.cu", "normals.cu"]
 NVCC_FLAGS = [
     "-O3", "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a", "-lineinfo", "--expt-relaxed-constexpr",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-fvisibility=hidden", "-DGSB200_BUILD",
 ]
+# per-file flags: the normal estimate evaluates normals.cuh without FMA contraction, exactly as the g++ host build
+# (-ffp-contract=off) of the test-suite does
+FILE_FLAGS = {"normals.cu": ["-fmad=false"]}
 
 
 def _deps_mtime() -> float:
@@ -41,7 +45,7 @@ def build(force: bool = False, ptxas_v: bool = False, verbose: bool = True, defi
 
     def compile_one(src):
         obj = os.path.join(BUILD, src.replace(".cu", tag + ".o"))
-        cmd = ["nvcc", *flags, "-c", os.path.join(CSRC, src), "-o", obj]
+        cmd = ["nvcc", *flags, *FILE_FLAGS.get(src, []), "-c", os.path.join(CSRC, src), "-o", obj]
         r = subprocess.run(cmd, capture_output=True, text=True)
         return src, obj, r
 

@@ -105,6 +105,22 @@ int launch_composite_bwd_sh(int C, bool fused, const CompositeArgs& a, cudaStrea
 // knn.cu: exact K nearest neighbours on a uniform grid (queries == nullptr: the points query themselves)
 int knn_device(gsb200_ctx* ctx, const float* points, uint32_t n, const float* queries, uint32_t nq, int K,
                int64_t* idx_out, float* d2_out, cudaStream_t st);
+// the grid behind it, built on `st` in the context's knn_* buffers: points sorted by cell, the cell table, and `order`
+// (order[s] = index of the point in sorted slot s, i.e. the points in cell order)
+struct KnnGrid;
+struct KnnPt;
+struct KnnIndex {
+  const KnnGrid* grid;
+  const KnnPt* sorted;
+  const int32_t* cell_start;
+  const int32_t* order;
+};
+int knn_build_index(gsb200_ctx* ctx, const float* points, uint32_t n, KnnIndex* out, cudaStream_t st);
+// normals.cu: per-point normals of the points' K-neighbourhoods (include/gsb200.h Part 7)
+int normals_device(gsb200_ctx* ctx, const float* points, uint32_t n, int K, int disambiguate, float* normals,
+                   int32_t* nbr_idx, cudaStream_t st);
+int normals_backward_device(const float* points, uint32_t n, int K, int disambiguate, const int32_t* nbr_idx,
+                            const float* grad_normals, float* grad_points, cudaStream_t st);
 
 // Opt a kernel in to more than 48 KB of dynamic shared memory.  Called before every launch: the attribute is per
 // (function, device) and the call is a few hundred ns -- cheaper than a lock-protected per-device cache, and correct

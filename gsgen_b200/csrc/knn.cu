@@ -177,15 +177,9 @@ static int knn_bits_for(uint32_t n) {
   return b;
 }
 
-int knn_device(gsb200_ctx* ctx, const float* points, uint32_t n, const float* queries, uint32_t nq, int K,
-               int64_t* idx_out, float* d2_out, cudaStream_t st) {
-  GSB_CHECK(K >= 1 && K <= kKnnMaxK, GSB200_ERR_UNSUPPORTED, "knn: K = %d outside [1, %d]", K, kKnnMaxK);
-  GSB_CHECK(n <= 0x7fffffffu / 4u, GSB200_ERR_INVALID, "knn: %u points exceed the int32 index range", n);
-  const bool self = (queries == nullptr);
-  if (self) { queries = points; nq = n; }
-  if (nq == 0) return GSB200_OK;
-  GSB_CHECK(points != nullptr || n == 0, GSB200_ERR_INVALID, "knn: points is NULL");
-  GSB_CHECK(idx_out != nullptr, GSB200_ERR_INVALID, "knn: idx_out is NULL");
+// The grid over `n` points on `st` (stats -> grid -> cell keys -> radix sort -> gather -> cell table), in the
+// context's knn_* buffers.  Shared by the neighbour search below and the normal estimate (normals.cu).
+int knn_build_index(gsb200_ctx* ctx, const float* points, uint32_t n, KnnIndex* out, cudaStream_t st) {
   // the cell table is sized on the host from N alone (the grid itself is chosen on the device)
   const uint32_t max_cells = 4u * n + 64u;
   int rc;
@@ -228,10 +222,30 @@ int knn_device(gsb200_ctx* ctx, const float* points, uint32_t n, const float* qu
   }
   k_knn_cells<<<(max_cells + 1 + 255) / 256, 256, 0, st>>>(n, k1, grid, ctx->knn_cells.as<int32_t>());
   GSB_LAUNCH_CHECK();
-  const int32_t* order = self ? v1 : nullptr;
+  out->grid = grid;
+  out->sorted = ctx->knn_pts.as<KnnPt>();
+  out->cell_start = ctx->knn_cells.as<int32_t>();
+  out->order = v1;
+  return GSB200_OK;
+}
+
+int knn_device(gsb200_ctx* ctx, const float* points, uint32_t n, const float* queries, uint32_t nq, int K,
+               int64_t* idx_out, float* d2_out, cudaStream_t st) {
+  GSB_CHECK(K >= 1 && K <= kKnnMaxK, GSB200_ERR_UNSUPPORTED, "knn: K = %d outside [1, %d]", K, kKnnMaxK);
+  GSB_CHECK(n <= 0x7fffffffu / 4u, GSB200_ERR_INVALID, "knn: %u points exceed the int32 index range", n);
+  const bool self = (queries == nullptr);
+  if (self) { queries = points; nq = n; }
+  if (nq == 0) return GSB200_OK;
+  GSB_CHECK(points != nullptr || n == 0, GSB200_ERR_INVALID, "knn: points is NULL");
+  GSB_CHECK(idx_out != nullptr, GSB200_ERR_INVALID, "knn: idx_out is NULL");
+  KnnIndex ix;
+  int rc;
+  if ((rc = knn_build_index(ctx, points, n, &ix, st))) return rc;
+  const int32_t* order = self ? ix.order : nullptr;
   const unsigned qblocks = (nq + 127) / 128;
-  const KnnPt* sp = ctx->knn_pts.as<KnnPt>();
-  const int32_t* cs = ctx->knn_cells.as<int32_t>();
+  const KnnGrid* grid = ix.grid;
+  const KnnPt* sp = ix.sorted;
+  const int32_t* cs = ix.cell_start;
   if (K <= 2) k_knn_query<2><<<qblocks, 128, 0, st>>>(nq, queries, order, grid, sp, cs, K, idx_out, d2_out);
   else if (K <= 4) k_knn_query<4><<<qblocks, 128, 0, st>>>(nq, queries, order, grid, sp, cs, K, idx_out, d2_out);
   else if (K <= 8) k_knn_query<8><<<qblocks, 128, 0, st>>>(nq, queries, order, grid, sp, cs, K, idx_out, d2_out);

@@ -24,6 +24,13 @@
 
 #include "gsb200_math.cuh"
 
+// (GSB_HD is `static` on the host, which member functions cannot be)
+#if defined(__CUDACC__)
+#define GSB_HD_MEMBER __host__ __device__ __forceinline__
+#else
+#define GSB_HD_MEMBER inline
+#endif
+
 namespace gsb {
 
 constexpr int kKnnMaxK = 32;
@@ -158,14 +165,12 @@ template <int K> GSB_HD void knn_insert(float (&bd)[K], int32_t (&bi)[K], float 
   }
 }
 
-// The K nearest points of (qx, qy, qz).  pts: the n points sorted by cell id; cell_start[c] .. cell_start[c+1]: the
-// points of cell c (cell_start has G.cells + 1 entries).  On return bd / bi hold the neighbours in ascending order;
-// slots beyond the number of points are (+inf, -1).  Returns the number of shells visited (statistics).
-template <int K>
-GSB_HD int knn_query(const KnnGrid& G, const KnnPt* pts, const int32_t* cell_start, float qx, float qy, float qz,
-                     float (&bd)[K], int32_t (&bi)[K]) {
-#pragma unroll
-  for (int j = 0; j < K; ++j) { bd[j] = INFINITY; bi[j] = -1; }
+// The shell walk of the search.  pts: the n points sorted by cell id; cell_start[c] .. cell_start[c+1]: the points of
+// cell c (cell_start has G.cells + 1 entries).  L: the K best so far -- L.insert(d, i) offers a candidate, L.kth() is
+// the current K-th best distance (+inf while fewer than K are known).  Returns the number of shells visited.
+template <class List>
+GSB_HD int knn_walk(const KnnGrid& G, const KnnPt* pts, const int32_t* cell_start, float qx, float qy, float qz,
+                    List& L) {
   const float q[3] = {qx, qy, qz};
   int c[3];
 #pragma unroll
@@ -193,7 +198,7 @@ GSB_HD int knn_query(const KnnGrid& G, const KnnPt* pts, const int32_t* cell_sta
           const int s0 = cell_start[row + xa], s1 = cell_start[row + xb + 1];
           for (int s = s0; s < s1; ++s) {
             const KnnPt p = pts[s];
-            knn_insert<K>(bd, bi, knn_dist2(p.x, p.y, p.z, qx, qy, qz), p.i);
+            L.insert(knn_dist2(p.x, p.y, p.z, qx, qy, qz), p.i);
           }
         }
       }
@@ -207,9 +212,57 @@ GSB_HD int knn_query(const KnnGrid& G, const KnnPt* pts, const int32_t* cell_sta
       if (c[a] + r < G.g[a] - 1) dmin = fminf(dmin, (G.lo[a] + (float)(c[a] + r + 1) * G.h) - q[a]);
     }
     const float safe = dmin - G.slack;
-    if (safe > 0.f && bd[K - 1] < safe * safe) break;  // strict: an uncovered point cannot even tie
+    if (safe > 0.f && L.kth() < safe * safe) break;  // strict: an uncovered point cannot even tie
   }
   return r + 1;
 }
+
+// the K best in registers (sorted insert network of knn_insert)
+template <int K>
+struct KnnRegList {
+  float (&bd)[K];
+  int32_t (&bi)[K];
+  GSB_HD_MEMBER void insert(float d, int32_t i) { knn_insert<K>(bd, bi, d, i); }
+  GSB_HD_MEMBER float kth() const { return bd[K - 1]; }
+};
+
+// The K nearest points of (qx, qy, qz) (see knn_walk).  On return bd / bi hold the neighbours in ascending order;
+// slots beyond the number of points are (+inf, -1).  Returns the number of shells visited (statistics).
+template <int K>
+GSB_HD int knn_query(const KnnGrid& G, const KnnPt* pts, const int32_t* cell_start, float qx, float qy, float qz,
+                     float (&bd)[K], int32_t (&bi)[K]) {
+#pragma unroll
+  for (int j = 0; j < K; ++j) { bd[j] = INFINITY; bi[j] = -1; }
+  KnnRegList<K> L{bd, bi};
+  return knn_walk(G, pts, cell_start, qx, qy, qz, L);
+}
+
+// The same K best as a strided list in memory (slot j at d[j * S], i[j * S]; shared memory on the device, where K
+// pairs would not fit in registers): insertion by shifting from the end, the order of knn_insert.
+template <int K, int S>
+struct KnnStridedList {
+  float* d;
+  int32_t* i;
+  float wd;    // the K-th best, cached
+  int32_t wi;
+  GSB_HD_MEMBER void init() {
+    for (int j = 0; j < K; ++j) { d[j * S] = INFINITY; i[j * S] = -1; }
+    wd = INFINITY; wi = -1;
+  }
+  GSB_HD_MEMBER void insert(float dd, int32_t ii) {
+    if (!(dd < wd || (dd == wd && ii < wi))) return;
+    int j = K - 1;
+    while (j > 0) {
+      const float pd = d[(j - 1) * S];
+      const int32_t pi = i[(j - 1) * S];
+      if (!(dd < pd || (dd == pd && ii < pi))) break;
+      d[j * S] = pd; i[j * S] = pi;
+      --j;
+    }
+    d[j * S] = dd; i[j * S] = ii;
+    wd = d[(K - 1) * S]; wi = i[(K - 1) * S];
+  }
+  GSB_HD_MEMBER float kth() const { return wd; }
+};
 
 }  // namespace gsb

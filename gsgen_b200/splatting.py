@@ -18,7 +18,8 @@ The trainer loop of the reference (`trainer.py:575-617`) then reads:
     renderer.optimizer.zero_grad()
 
 Only the default configuration of the reference is covered: exp / sigmoid / sigmoid activations, RGB colours (no PBR
-shading, no learned normals), a constant or per-pixel background.  `render_fn` exists so that this host logic can be
+shading, no learned normals), a constant or per-pixel background, and `normal_as_rgb` (normals estimated from the means,
+rendered as colours: gsgen_b200/normals.py).  `render_fn` exists so that this host logic can be
 exercised without a GPU (the test-suite plugs in the CPU oracle); the default is the CUDA path and there is no
 fallback.
 """
@@ -27,6 +28,7 @@ from __future__ import annotations
 from typing import Callable, Dict, Optional, Sequence
 
 import torch
+import torch.nn.functional as F
 
 from .store import GaussianStore, quat_to_rotmat
 
@@ -132,6 +134,22 @@ class GaussianSplattingRenderer:
     bg = property(lambda self: self.background)                                 # the attribute name the reference uses
 
     @property
+    def normal(self) -> torch.Tensor:
+        """:1189-1196, the `normal_type: "estimated"` branch: one normal per Gaussian from the means,
+        `estimate_normal(self.mean, **cfg.normal)` (the function's defaults where cfg has no `normal` block); the
+        gradient reaches `mean` through it.  `knn_fn` (CPU test-suite) feeds it as it feeds the compactness rules."""
+        from .normals import estimate_normal
+
+        c = _get(self.cfg, "normal", None)
+        return estimate_normal(self.mean, neighborhood_size=_get(c, "neighborhood_size", 50),
+                               disambiguate_directions=_get(c, "disambiguate_directions", True), knn=self.store.knn_fn)
+
+    def update_normal(self) -> torch.Tensor:
+        """:1185-1187.  The reference assigns to the read-only `normal` property there (an AttributeError on an
+        nn.Module, so its normal_as_rgb path never ran); here it returns the estimate the property defines."""
+        return self.normal
+
+    @property
     def is_densifying(self) -> bool:
         """:163-169"""
         d = _get(self.cfg, "densify", None)
@@ -210,6 +228,11 @@ class GaussianSplattingRenderer:
                 raise RuntimeError(f"overrides for unknown fields {unknown}")
             act = {f: (overrides[f] if f in overrides else getattr(self, f)) for f in FIELDS}
             leaves, raw = (act["mean"], act["qvec"], act["svec"], act["alpha"], act["color"]), False
+        return self._render(leaves, raw, raw, c2w, camera_info, use_bg, rgb_only, return_T)
+
+    def _render(self, leaves, raw: bool, sink: bool, c2w, camera_info, use_bg, rgb_only, return_T):
+        """one view of (mean, qvec, svec, alpha, color): raw leaves (activations in the kernels) or activated values;
+        `sink`: gradients go straight into the arena's flat gradient buffer (only when every leaf IS an arena leaf)"""
         out = self._render_fn(
             leaves[0], leaves[1], leaves[2], leaves[3], c2w, camera_info, color=leaves[4],
             bg=self._bg_image(camera_info, c2w, use_bg), rgb_only=rgb_only, raw_params=raw,
@@ -218,7 +241,7 @@ class GaussianSplattingRenderer:
             skip_frustum_culling=_get(self.cfg, "skip_frustum_culling", False),
             depth_detach=_get(self.cfg, "depth_detach", True),
             # (the flat gradient sink holds gradients w.r.t. the RAW leaves: only the raw-leaf path may write into it)
-            grad_sink=self.store.grad_views if (self.training and raw) else None,
+            grad_sink=self.store.grad_views if (self.training and sink) else None,
             # one library context per in-flight view: the views of a batch are all rendered before ONE loss.backward()
             # (trainer.py:575-599), and a context keeps a view's binning + splat records until its backward has run
             slot=len(self._pending) if self.training else 0)
@@ -240,7 +263,22 @@ class GaussianSplattingRenderer:
     def __call__(self, batch, use_bg: bool = True, rgb_only: bool = False):
         """forward(batch) (:1426-1460): batch["c2w"] [bs,3,4] (host or device), batch["camera_info"] list"""
         c2ws, infos = batch["c2w"], batch["camera_info"]
-        return stack_dicts([self.render_one(c2ws[i], infos[i], use_bg, rgb_only) for i in range(len(infos))])
+        if not _get(self.cfg, "normal_as_rgb", False):
+            return stack_dicts([self.render_one(c2ws[i], infos[i], use_bg, rgb_only) for i in range(len(infos))])
+        # cfg.normal_as_rgb (:1427-1430, :1462-1463): the normals, estimated once per batch, replace the colours of
+        # every view; the composited colour is normalised back to a direction and mapped to [0, 1]
+        # The views run on the raw arena leaves with the colour leaf replaced by logit((n + 1) / 2) -- the kernels'
+        # sigmoid gives the colour back to fp32 rounding (logit clamped at 1e-6 from 0 and 1, where a normal component
+        # is exactly -1 or 1) -- and without the flat gradient sink, so autograd takes the colour gradient to the
+        # normals and from there to `mean`, and the colour leaf gets none.  Same image as
+        # render_one(overrides={"color": (n + 1) / 2}) to ~1e-6, on the raw-leaf path every render_fn provides.
+        p = self.store.params
+        col = torch.logit((self.update_normal() + 1.0) * 0.5, eps=1e-6)
+        leaves = (p["mean"], p["qvec"], p["svec"], p["alpha"], col)
+        out = stack_dicts([self._render(leaves, True, False, c2ws[i], infos[i], use_bg, rgb_only, False)
+                           for i in range(len(infos))])
+        out["rgb"] = (F.normalize(out["rgb"], dim=-1, eps=1e-6) + 1.0) / 2.0
+        return out
 
     forward = __call__
 

@@ -356,6 +356,28 @@ int gsb200_rows_unpack(gsb200_ctx* ctx, float* flat, const float* packed, const 
 int gsb200_knn(gsb200_ctx* ctx, const float* points, uint32_t n_points, const float* queries, uint32_t n_queries,
                int32_t K, int64_t* idx, float* dist2, gsb200_stream stream);
 
+/* ================================================================================================
+ * Part 7 -- per-point normals of a point cloud (the Gaussian means): utils/ops.py:62-72 estimate_normal, i.e.
+ * pytorch3d.ops.estimate_pointcloud_normals(points, K, disambiguate_directions), used by gs/gaussian_splatting.py
+ * for cfg.normal_as_rgb and by utils/relight.py.  For every point: its K nearest points (itself included, the exact
+ * search of Part 6), C = (1/K) sum_k (x_k - mu)(x_k - mu)^T, the unit eigenvector of C's smallest eigenvalue; with
+ * disambiguate != 0 it is negated when fewer than K/2 neighbours x_k satisfy n . (x_k - p) > 0.  A zero or non-finite
+ * covariance gives (0, 0, 1) before that flip.  1 <= K <= 64 and K <= n_points (GSB200_ERR_UNSUPPORTED /
+ * GSB200_ERR_INVALID otherwise).
+ *
+ * gsb200_estimate_normals: points [n,3] fp32 -> normals [n,3] fp32; nbr_idx [n,K] int32 receives the neighbour
+ * indices (ascending distance, ties by index) for the backward, or is NULL (then nothing of size [n,K] is written).
+ * gsb200_estimate_normals_backward: ADDS dL/dpoints to grad_points [n,3] for dL/dnormals = grad_normals [n,3], with the
+ * forward's neighbour sets (nbr_idx) and signs held constant (the sign is recomputed: pass the forward's disambiguate).
+ * An eigen gap |lam_0 - lam_j| <= 1e-6 max(lam_2, 1e-30) contributes zero instead of inf / NaN.  Atomic accumulation:
+ * not bitwise reproducible.  Both run on `stream` without synchronising.
+ * ============================================================================================== */
+int gsb200_estimate_normals(gsb200_ctx* ctx, const float* points, uint32_t n_points, int32_t K, int32_t disambiguate,
+                            float* normals, int32_t* nbr_idx, gsb200_stream stream);
+int gsb200_estimate_normals_backward(gsb200_ctx* ctx, const float* points, uint32_t n_points, int32_t K,
+                                     int32_t disambiguate, const int32_t* nbr_idx, const float* grad_normals,
+                                     float* grad_points, gsb200_stream stream);
+
 #if defined(__GNUC__)
 #pragma GCC visibility pop
 #endif
